@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR   (also writes the patch of the last timed step as DIR/*.npy: patch_arrays)
 
 Workload (BASELINE.json `metric`: "ops/sec applied (1M-op text trace)"; SURVEY.md §8d C3): a makeText
 change plus 10 actors x 100 000 single-op changes (70 % insert / 30 % delete, merge every 100 changes)
@@ -35,6 +36,8 @@ import subprocess
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -183,8 +186,9 @@ def bind_to_gpu_numa_node(local):
         return None
 
 
-def measure(args, wl_name, rank, world, local, lib, torch, dist, full):
-    """K timed steps of one workload. Returns the pieces of the JSON line."""
+def measure(args, wl_name, rank, world, local, lib, torch, dist, full, keep_patch=False):
+    """K timed steps of one workload. Returns the pieces of the JSON line (with keep_patch, also the bytes of the flat
+    patch the last timed step returned)."""
     import numpy as np
     from automerge_classic_b200 import tracegen
     from automerge_classic_b200.engine import GpuBackendDoc, _ErrStruct
@@ -207,7 +211,7 @@ def measure(args, wl_name, rank, world, local, lib, torch, dist, full):
     L.amg_reserve(doc.h, C.c_size_t(nbytes + (1 << 20)), C.byref(err))
     state = {}
 
-    def step(ptr):
+    def step(ptr, keep=False):
         lib.check(L.amg_reset(doc.h, C.byref(err)), err)
         pp = C.c_void_p()
         torch.cuda.synchronize()
@@ -218,14 +222,16 @@ def measure(args, wl_name, rank, world, local, lib, torch, dist, full):
         dt = time.perf_counter() - t0
         lib.check(rc, err)
         n = C.c_size_t()
-        L.amg_patch_bytes(pp, C.byref(n))
+        p = L.amg_patch_bytes(pp, C.byref(n))
+        if keep:
+            state['patch'] = bytes((C.c_uint8 * n.value).from_address(p))
         L.amg_patch_free(pp)
         return dt, doc.timings(), n.value
 
-    def timed(ptr, steps):
+    def timed(ptr, steps, keep_last=False):
         wall, dev, ph, pb = [], [], None, 0
-        for _ in range(steps):
-            dt, ph, pb = step(ptr)
+        for i in range(steps):
+            dt, ph, pb = step(ptr, keep_last and i == steps - 1)
             wall.append(dt)
             dev.append(sum(ph[0:12]) / 1e3)   # CUDA events on the engine's stream, first to last kernel of the call
         return wall, dev, ph, pb
@@ -245,7 +251,7 @@ def measure(args, wl_name, rank, world, local, lib, torch, dist, full):
     if world > 1:
         dist.barrier()
     launches0 = doc.launches()
-    wall, dev_e2e, last_ph, patch_bytes = timed(pinned.data_ptr(), args.steps)
+    wall, dev_e2e, last_ph, patch_bytes = timed(pinned.data_ptr(), args.steps, keep_last=keep_patch)
     torch.cuda.synchronize()
     sampler.mark()
     if world > 1:
@@ -258,7 +264,8 @@ def measure(args, wl_name, rank, world, local, lib, torch, dist, full):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         t_wall, t_dev = float(tt[0]), float(tt[1])
     res = {'trace': trace, 'nbytes': nbytes, 'desc': desc, 't_wall': t_wall, 't_dev': t_dev, 'wall_steps': wall, 'dev_steps': dev_res, 'last_ph': last_ph, 'ph_res': ph_res,
-           'patch_bytes': patch_bytes, 'launches': int(launches), 'call_ms': state['call_ms'], 'clocks': sampler.summary(), 'doc': doc, 'pinned': pinned, 'offs': offs, 'offs_pinned': offs_pinned}
+           'patch_bytes': patch_bytes, 'launches': int(launches), 'call_ms': state['call_ms'], 'clocks': sampler.summary(), 'doc': doc, 'pinned': pinned, 'offs': offs, 'offs_pinned': offs_pinned,
+           'patch': state.get('patch')}
     if not full:
         del doc
     return res
@@ -291,6 +298,84 @@ def ptr_array_e2e(trace, lib, torch, local, steps):
     return sum(times) / len(times)
 
 
+DUMP_BUDGET = 64_000_000   # bytes --dump-outputs writes at most
+DUMP_SEED = 20261017
+
+
+def _gather(buf, off, length):
+    """buf[off[i]:off[i] + length[i]] of every row, back to back."""
+    length = length.astype(np.int64)
+    idx = np.repeat(off.astype(np.int64) - (np.cumsum(length) - length), length) + np.arange(int(length.sum()))
+    return buf[idx]
+
+
+def _split_ids(name, ids):
+    """opIds are (counter << 16 | actor index): two columns, each exact in float64."""
+    ids = ids.astype(np.uint64)
+    return {name + '_ctr': ids >> np.uint64(16), name + '_actor': ids & np.uint64(0xffff)}
+
+
+def patch_arrays(raw, budget=DUMP_BUDGET, seed=DUMP_SEED):
+    """The flat patch of include/amgpu.h (what amg_apply_changes_packed hands its caller) as named float64 / float32 arrays:
+    the header counts, actor table, clock, heads, and the map-property and list-edit records column by column. Payload
+    bytes (keys, values) are gathered per record instead of their offsets in the patch buffer, so that two builds that
+    compute the same patch dump the same arrays however they lay the buffer out. When the records would take more than
+    `budget` bytes, a fixed seeded sample of them is kept, in order; their record numbers are the `*_row` arrays."""
+    from automerge_classic_b200.engine import FlatPatch
+    fp = FlatPatch(raw)
+    h = fp.hdr
+    buf = np.frombuffer(raw, dtype=np.uint8)
+    out = {'header': np.array([fp.max_op, fp.pending, int(h[3]), int(h[4]), int(h[8]), int(h[10]), int(h[12]), int(h[14]), int(h[16])], dtype=np.float64)}
+    ids = [bytes.fromhex(a) for a in fp.actors]
+    actors = np.full((len(ids), max([len(a) for a in ids] + [0])), -1.0)
+    for i, a in enumerate(ids):
+        actors[i, :len(a)] = np.frombuffer(a, dtype=np.uint8)
+    out['actors'] = actors
+    out['clock'] = np.frombuffer(raw, dtype='<u8', count=2 * int(h[10]), offset=int(h[9])).reshape(-1, 2).astype(np.float64)
+    out['deps'] = buf[int(h[11]):int(h[11]) + 32 * int(h[12])].reshape(-1, 32).astype(np.float64)
+
+    p, e = fp.props, fp.edits
+    p_action, p_flags = p['flags'] >> 8, p['flags']
+    p_counter = (p_action == 1) & (p_flags & 2 != 0)
+    p_vlen = np.where((p_action == 1) & (p_flags & 3 == 0), p['valLen'] >> 4, 0)
+    props = {**_split_ids('obj', p['obj']), **_split_ids('op', p['opId']), 'key_len': p['keyLen'], 'flags': p_flags, 'val_len': p['valLen'],
+             'counter': np.where(p_counter, (p['valOff'].astype(np.uint64) | (p['pad'].astype(np.uint64) << np.uint64(32))).view(np.int64), 0)}
+    e_kind = e['kind']
+    e_counter = e_kind & 0x1000 != 0
+    e_vlen = np.where((e_kind & 0xff != 1) & (e_kind >> 16 == 1) & ~e_counter, e['valLen'] >> 4, 0)
+    edits = {**_split_ids('obj', e['obj']), **_split_ids('op', e['opId']), **_split_ids('elem', fp.edit_elem), 'index': e['index'], 'kind': e_kind,
+             'val_len': e['valLen'], 'counter': np.where(e_counter, (e['valLen'].astype(np.uint64) | (e['valOff'].astype(np.uint64) << np.uint64(32))).view(np.int64), 0)}
+    # payload bytes go out as float32 (4 bytes each), record columns as float64 (8 bytes each, plus the record number)
+    tables = [('props', props, [('key', p['keyOff'], p['keyLen']), ('value', p['valOff'], p_vlen)]),
+              ('edits', edits, [('value', e['valOff'], e_vlen)])]
+    cost = [8 * (len(cols) + 1) + 4 * sum(ln.astype(np.int64) for _, _, ln in pays) for _, cols, pays in tables]
+    room = budget - sum(a.nbytes for a in out.values()) - 128 * (len(out) + sum(len(c) + 1 + len(pl) for _, c, pl in tables))
+    rng = np.random.default_rng(seed)
+    # the smaller table first: it keeps every record if it fits its half of the room, the other table gets the rest
+    for left, k in enumerate(sorted(range(len(tables)), key=lambda k: int(cost[k].sum()))):
+        (name, cols, pays), c = tables[k], cost[k]
+        rows = np.arange(len(c))
+        if int(c.sum()) > room // (len(tables) - left):
+            order = rng.permutation(len(c))
+            rows = np.sort(order[:np.searchsorted(np.cumsum(c[order]), room // (len(tables) - left), side='right')])
+        room -= int(c[rows].sum())
+        out[name + '_row'] = rows.astype(np.float64)
+        for col, v in cols.items():
+            out['%s_%s' % (name, col)] = np.asarray(v)[rows].astype(np.float64)
+        for pay, off, ln in pays:
+            out['%s_%s_bytes' % (name, pay)] = _gather(buf, off[rows], ln[rows]).astype(np.float32)
+    return out
+
+
+def dump_outputs(raw, out_dir):
+    """Writes the arrays of patch_arrays that have elements (a workload without list edits, or a patch whose map entries
+    carry no value bytes, has nothing to compare there)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in patch_arrays(raw).items():
+        if a.size:
+            np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def cpu_sample(wl_name, sample_ops):
     import oracle
     from automerge_classic_b200 import tracegen
@@ -319,6 +404,8 @@ def main():
     ap.add_argument('--workload', default='C3', choices=sorted(WORKLOADS))
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='headline figures only (no other routes / workloads / pointer-array entry)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the patch the last timed step returned as DIR/<name>.npy (see patch_arrays; '
+                                                         'at most 64 MB, a fixed seeded sample of the records if the patch is larger)')
     args = ap.parse_args()
     rank, world, local = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1)), int(os.environ.get('LOCAL_RANK', 0))
     if args.impl == 'reference':
@@ -343,7 +430,9 @@ def main():
     L = lib.L
     err = _ErrStruct()
 
-    m = measure(args, args.workload, rank, world, local, lib, torch, dist, full=True)
+    m = measure(args, args.workload, rank, world, local, lib, torch, dist, full=True, keep_patch=bool(args.dump_outputs))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(m['patch'], args.dump_outputs)
     trace, doc, nbytes = m['trace'], m['doc'], m['nbytes']
     t_wall, t_dev, last_ph = m['t_wall'], m['t_dev'], m['last_ph']
     total_ops = trace.n_ops * world

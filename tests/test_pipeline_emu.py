@@ -219,3 +219,46 @@ def test_deflate_fuzz_emu(emu_doc, oracle_mod):
 def test_apply_corrupted_emu(emu_doc, oracle_mod):
     both, refused, engine_only = parity_checks.check_apply_corrupted(emu_doc, oracle_mod, 40)
     assert both > 5 and refused > 5
+
+
+DUMP_SCRIPT = r'''
+import os, sys, numpy as np
+sys.path.insert(0, %(root)r)
+import bench                     # (bench.py sends file descriptor 1 to stderr: run in a process of its own)
+raw = open(%(raw)r, 'rb').read()
+bench.dump_outputs(raw, os.path.join(%(out)r, 'full'))
+for d in ('a', 'b'):
+    os.makedirs(os.path.join(%(out)r, d))
+    for name, a in bench.patch_arrays(raw, budget=20000).items():
+        np.save(os.path.join(%(out)r, d, name + '.npy'), a)
+'''
+
+
+def test_bench_dump_outputs_emu(emu_doc, tmp_path):
+    """bench.py --dump-outputs: the arrays carry the flat patch's records and value bytes; under a smaller budget they are a
+    seeded sample of the records that fits it and is the same on every run."""
+    import sys
+    import numpy as np
+    from automerge_classic_b200 import tracegen
+    t = tracegen.generate('C3', 3000, 3)
+    fp = emu_doc().apply_packed_flat(t.blob, t.offsets, t.n_changes)
+    (tmp_path / 'patch.bin').write_bytes(fp.raw)
+    script = tmp_path / 'dump.py'
+    script.write_text(DUMP_SCRIPT % {'root': os.path.dirname(HERE), 'raw': str(tmp_path / 'patch.bin'), 'out': str(tmp_path)})
+    out = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stderr[-2000:]
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(tmp_path, d, f)) for f in os.listdir(tmp_path / d)}
+    full, a, b = load('full'), load('a'), load('b')
+    assert all(v.dtype in (np.float32, np.float64) and v.size for v in full.values())
+    assert 'props_key_bytes' in full and 'props_value_bytes' not in full   # the makeText entry has a key and no value bytes
+    assert full['header'][0] == fp.max_op and np.array_equal(full['edits_row'], np.arange(len(fp.edits)))
+    assert np.array_equal((full['edits_op_ctr'] * 65536 + full['edits_op_actor']).astype(np.uint64), fp.edits['opId'])
+    text = [o for c in fp.to_patch(False)['diffs']['props'].values() for o in c.values()][0]
+    chars = ''.join(v for e in text['edits'] for v in ([e['value']['value']] if e['action'] == 'insert' else e.get('values', [])))
+    assert bytes(full['edits_value_bytes'].astype(np.uint8)).decode() == chars
+    assert sum(os.path.getsize(os.path.join(tmp_path, 'a', f)) for f in os.listdir(tmp_path / 'a')) <= 20000
+    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+    rows = a['edits_row'].astype(np.int64)
+    assert 0 < len(rows) < len(fp.edits) and np.array_equal(a['edits_index'], fp.edits['index'][rows])
